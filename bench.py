@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- stage-1 structural indexing throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--check]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--check] [--dump-outputs DIR]
 
 One "step" = one stage-1 pass (structural indexing + UTF-8 validation) over one batch of synthetic input per GPU.
 
@@ -32,6 +32,9 @@ The JSON line carries:
   cpu_baseline  the reference's own CPU stage 1 (oracle/_ref, the unmodified reference) on this box's host cores:
             pre-spawned threads, one private copy of the document per thread; all cores and one core
 `--impl reference` times that CPU implementation as its own arm (rank 0 only).
+
+`--dump-outputs DIR` (stage1_64m) writes what the last timed step returned, as float64 .npy files under DIR (see
+dump_outputs), so that two builds can be compared output for output: the inputs are seeded, the same on every run.
 """
 import argparse
 import ctypes as C
@@ -46,12 +49,14 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # bench.py writes nothing into the tree it runs from, bytecode caches of its modules included
 
 DOC_BYTES = 64 << 20
 ROTATE = 4  # distinct 64 MiB inputs used round-robin: 256 MiB > 126 MB of L2, so no step finds its input in L2
 METRIC = "stage1 GB/s (bytes in / s) vs HBM roofline at 1/2/4/8 B200; CPU ref GB/s"
 UNIT = "GB/s"
 PLUGIN = os.path.join(ROOT, "simdjson_b200", "plugin", "libsimdjson_b200.so")
+DUMP_LIMIT = 64_000_000  # bytes of --dump-outputs in all, .npy headers included
 KERNEL_SOURCES = ["sjb200_scan4.cuh", "sjb200_bits.cuh", "sjb200_simt.cuh", "sjb200_params.h", "sjb200_kernels.cu", "sjb200_utf8.cuh"]
 
 
@@ -303,6 +308,26 @@ def cpu_baseline(doc, steps=3):
     return {"value": round((16 << 20) / dt / 1e9, 3), "unit": UNIT, "cores": 1, "kind": "port", "sample": "scalar C port, 16 MiB prefix, one pass"}
 
 
+def dump_sample(n, k):
+    """positions of the k of n index words that --dump-outputs keeps when all n do not fit: fixed by the seed, sorted"""
+    return np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+
+
+def dump_outputs(out_dir, rank, world, scalars, words):
+    """--dump-outputs: the last timed step's results (scalars: name -> value) and index words, as float64 .npy files (exact
+    for 32-bit values), named rank<r>_<name>.npy when world > 1.  The index words go out whole when they fit this rank's
+    share of DUMP_LIMIT, else as words[dump_sample(len(words), cap)]; len(words) is n_structural_indexes + 3 at one rank
+    and count at several."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = (DUMP_LIMIT // world - 4096) // 8  # float64 words; 4 KiB covers the .npy headers of this rank's files
+    if len(words) > cap:
+        words = words[dump_sample(len(words), cap)]
+    arrays = dict(scalars, structural_indexes=words)
+    prefix = f"rank{rank}_" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, dtype=np.float64).reshape(-1))
+
+
 # =============================================================================== reference arm
 def run_reference(args, rank, world):
     """the reference's own CPU stage 1 (oracle/_ref = unmodified reference, compiled in the build container) on this box's
@@ -461,6 +486,16 @@ def run_ours(args, rank, world):
     ms_per_step = total_ms / args.steps
     value = world * DOC_BYTES / (ms_per_step * 1e-3) / 1e9
 
+    if args.dump_outputs:
+        last = (args.steps - 1) % ROTATE  # the input (and index buffer) of the last timed step
+        got = d_idxs[last].cpu().numpy().view(np.uint32)
+        if world == 1:
+            n = results[last][0]
+            dump_outputs(args.dump_outputs, rank, world, {"n_structural_indexes": n}, got[: n + 3])
+        else:
+            count, base, _state_in, _rescanned, total = results[last]
+            dump_outputs(args.dump_outputs, rank, world, {"count": count, "base": base, "total_count": total}, got[:count])
+
     # ---- parity gate: the output every distinct input left behind in the timed region, against the oracle
     parity_ok, checked, rescans = True, 0, 0
     first_words = None
@@ -556,7 +591,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="stage1_64m", choices=["stage1_64m", "jsonexamples", "ndjson_1g", "utf8_minify_256m", "concat_8g", "tokens_64m"])
     ap.add_argument("--check", action="store_true", help="parity gate of the multi-rank path on adversarial cuts")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.check or args.config != "stage1_64m"):
+        ap.error("--dump-outputs writes the outputs of --impl ours --config stage1_64m")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     if args.impl == "reference":

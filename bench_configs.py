@@ -65,8 +65,13 @@ def _roofline(algo_bytes, kms, kernel):
             "peak_source": src, "kernel_ms": round(kms, 5), "algorithmic_bytes": int(algo_bytes), "kernel_src_sha16": B.kernel_source_hash()}
 
 
+def _warmup(args):
+    """untimed passes before the timed ones, the same floor as bench.py's default config"""
+    return max(3, args.warmup)
+
+
 def _line(args, world, value, ms_per_step, config, extra):
-    d = {"metric": B.METRIC, "value": round(value, 2), "unit": B.UNIT, "n_gpus": world, "steps": args.steps, "warmup": max(3, args.warmup), "ms_per_step": round(ms_per_step, 5),
+    d = {"metric": B.METRIC, "value": round(value, 2), "unit": B.UNIT, "n_gpus": world, "steps": args.steps, "warmup": _warmup(args), "ms_per_step": round(ms_per_step, 5),
          "higher_is_better": True, "scaling": "strong" if world > 1 else "weak", "vs_baseline": None, "dtype": "u8", "data": "synthetic", "config": config}
     d.update(extra)
     return d
@@ -82,15 +87,12 @@ def run_jsonexamples(args, rank, world):
     rc, parser = sj.get_active_implementation(local).create_dom_parser_implementation(4 << 20)
     parser.set_option("time_kernel", 1)
     files, ok = [], True
-    steps = max(10, args.steps)
+    steps = args.steps
     for name, mode in (("twitter.json", 0), ("citm_catalog.json", 0), ("amazon_cellphones.ndjson", 2)):
-        path = os.path.join(O.JSONEXAMPLES, name)
-        if not os.path.exists(path):
-            continue
-        data = np.fromfile(path, dtype=np.uint8)
+        data = np.frombuffer(O.jsonexample(name), dtype=np.uint8).copy()
         d = torch.from_numpy(data).to(dev)
         want = port.stage1(data, mode)
-        for _ in range(3):
+        for _ in range(_warmup(args)):
             parser.stage1_device(d, mode)
         parser.get_stat("kernel_ms_mean")
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -142,7 +144,7 @@ def run_ndjson(args, rank, world, total=1 << 30):
     stream = torch.cuda.Stream(device=dev)
     torch.cuda.set_stream(stream)
     comm = _connect(torch, dist, sharding, parser, rank, world, dev) if world > 1 else None
-    steps = max(3, min(args.steps, 20))
+    steps = args.steps
     last = None
 
     def one_pass():
@@ -155,7 +157,7 @@ def run_ndjson(args, rank, world, total=1 << 30):
             if rcs != 0:
                 raise RuntimeError("sharded scan failed: " + parser.last_cuda_error())
             last = (rcs, int(res.count), int(res.base), int(res.state_in), int(res.total_count), int(res.rescanned))
-    for _ in range(3):
+    for _ in range(_warmup(args)):
         one_pass()
     parser.get_stat("kernel_ms_mean")
     if world > 1:
@@ -206,7 +208,7 @@ def run_utf8_minify(args, rank, world, size=256 << 20):
     from simdjson_b200 import corpus
     O = B.oracle()
     port = O.Port()
-    steps = max(3, min(args.steps, 20))
+    steps, warm = args.steps, _warmup(args)
     rc, parser = sj.get_active_implementation(local).create_dom_parser_implementation(size)
     parser.set_option("time_kernel", 1)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
@@ -220,12 +222,12 @@ def run_utf8_minify(args, rank, world, size=256 << 20):
         ok = ok and parser.validate_utf8_device(bad) == 0
         del bad
     ts = []
-    for it in range(steps):
+    for it in range(warm + steps):
         flush.fill_(it)
         torch.cuda.synchronize()
         parser.validate_utf8_device(du)
         ts.append(parser.get_stat("kernel_ms"))
-    ums = float(np.mean(ts[1:]))
+    ums = float(np.mean(ts[warm:]))
     del du
     # ---- minify
     j = corpus.random_json(size, pretty_bias=0.8, utf8_rate=0.15).copy()
@@ -235,17 +237,17 @@ def run_utf8_minify(args, rank, world, size=256 << 20):
     rcm, dl = parser.minify_device(dj, dst)
     okm = rcm == werr and dl == len(wout) and torch.equal(dst[:dl].cpu(), torch.from_numpy(np.frombuffer(wout, dtype=np.uint8).copy()))
     ts = []
-    for it in range(steps):
+    for it in range(warm + steps):
         flush.fill_(it)
         torch.cuda.synchronize()
         parser.minify_device(dj, dst)
         ts.append(parser.get_stat("kernel_ms"))
-    mms = float(np.mean(ts[1:]))
+    mms = float(np.mean(ts[warm:]))
     ok = bool(ok and okm)
     line = _line(args, 1, size / (ums * 1e-3) / 1e9, ums,
                  {"workload": "validate_utf8 + minify on 256 MiB mixed-ASCII/UTF-8 synthetic, 1xB200 (BASELINE.json configs[3])", "bytes": size,
                   "l2": "a 256 MiB buffer is written between launches (cold L2)", "value_is": "validate_utf8 input GB/s (kernel); minify below"},
-                 {"parity": {"ok": ok, "against": "CPU oracle: verdict (valid + 3 corrupted copies), whole minified buffer"}, "gpu_launches": 2 * steps + 5,
+                 {"parity": {"ok": ok, "against": "CPU oracle: verdict (valid + 3 corrupted copies), whole minified buffer"}, "gpu_launches": 2 * (warm + steps) + 5,
                   "roofline": dict(_roofline(size, ums, "utf8v2_kernel"), kernel="sjb200::utf8v2_kernel (sjb200_utf8.cuh)"),
                   "minify": {"input_gbs": round(size / (mms * 1e-3) / 1e9, 1), "kept_fraction": round(dl / size, 4), "kernel_ms": round(mms, 5),
                              "roofline": dict(_roofline(size + dl, mms, "scan4_minify_kernel"), kernel="sjb200::scan4_minify_kernel (1 B read + kept bytes written per input byte)")},
@@ -265,7 +267,7 @@ def run_tokens(args, rank, world, size=64 << 20):
     from simdjson_b200 import corpus
     O = B.oracle()
     port = O.Port()
-    steps = max(3, min(args.steps, 20))
+    steps, warm = args.steps, _warmup(args)
     doc = corpus.random_json(size).copy()
     d = torch.from_numpy(doc).to(dev)
     rc, parser = sj.get_active_implementation(local).create_dom_parser_implementation(size)
@@ -281,7 +283,7 @@ def run_tokens(args, rank, world, size=64 << 20):
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
     stream = torch.cuda.current_stream()
     ts = []
-    for it in range(steps + 1):
+    for it in range(warm + steps):
         flush.fill_(it)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
@@ -290,7 +292,7 @@ def run_tokens(args, rank, world, size=64 << 20):
         e1.record(stream)
         torch.cuda.synchronize()
         ts.append(e0.elapsed_time(e1))
-    ms = float(np.mean(ts[1:]))
+    ms = float(np.mean(ts[warm:]))
     r = port.stage1(doc)
     t0 = time.time()
     want = port.tokens(doc, r.idx, r.n, strbuf_cap=cap)
@@ -305,7 +307,7 @@ def run_tokens(args, rank, world, size=64 << 20):
                   "bytes": size, "structurals": int(n), "strings": int(res.n_strings), "string_buf_bytes": int(res.string_bytes),
                   "l2": "a 256 MiB buffer is written between calls (cold L2)", "value_is": "document bytes per second through sjb200_tokens_dev (3 launches + the 24-byte result)",
                   "api": "sjb200_tokens_dev", "tok_stage": int(os.environ.get("SJB200_TOK_STAGE", "1"))},
-                 {"parity": {"ok": bool(ok), "against": "CPU oracle (sjo_tokens): every type, payload and string-buffer byte"}, "gpu_launches": 3 * (steps + 1),
+                 {"parity": {"ok": bool(ok), "against": "CPU oracle (sjo_tokens): every type, payload and string-buffer byte"}, "gpu_launches": 3 * (warm + steps),
                   "roofline": dict(_roofline(algo, ms, "token_scan_kernel"), kernel="sjb200::token_scan_kernel + tile_scan_kernel + string_write_kernel (sjb200_tape.cu), one call",
                                    note="the call's three launches together; strings are walked twice (length, then copy)"),
                   "cpu_baseline": {"value": round(size / cpu_s / 1e9, 3), "unit": B.UNIT, "cores": 1, "kind": "port", "sample": "sjo_tokens (oracle/sj_oracle.c) on the whole 64 MiB document, one call"},
@@ -323,7 +325,7 @@ def run_concat(args, rank, world, nshards=8, shard_target=1 << 30):
     port = O.Port()
     if nshards % world != 0:
         raise SystemExit("concat_8g needs 1, 2, 4 or 8 ranks")
-    unit = b"".join(open(os.path.join(O.JSONEXAMPLES, f), "rb").read() + b"\n" for f in ("twitter.json", "citm_catalog.json"))
+    unit = b"".join(O.jsonexample(f) + b"\n" for f in ("twitter.json", "citm_catalog.json"))
     unit_a = np.frombuffer(unit, dtype=np.uint8)
     reps = shard_target // len(unit)
     shard = np.tile(unit_a, reps)  # every shard is the same bytes: reps whole (twitter, citm) pairs, cut at a document boundary
@@ -337,7 +339,7 @@ def run_concat(args, rank, world, nshards=8, shard_target=1 << 30):
     torch.cuda.set_stream(stream)
     comm = _connect(torch, dist, sharding, parser, rank, world, dev) if world > 1 else sharding.Comm(parser, 0, 1)
     rounds = nshards // world
-    steps = max(2, min(args.steps, 5))
+    steps = args.steps
 
     def whole_job():
         """8 shards: `rounds` sharded passes of `world` shards each; 64-bit bases accumulate over the rounds on the host"""
@@ -349,7 +351,8 @@ def run_concat(args, rank, world, nshards=8, shard_target=1 << 30):
             out.append((q * world + rank, base + int(res.base), int(res.count), int(res.rescanned)))
             base += int(res.total_count)
         return out, base
-    whole_job()
+    for _ in range(_warmup(args)):
+        whole_job()
     parser.get_stat("kernel_ms_mean")
     if world > 1:
         dist.barrier()

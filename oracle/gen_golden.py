@@ -148,7 +148,7 @@ def main():
     # ---- whole-file digests for the reference's own corpora
     files = []
     for name, mode in [("twitter.json", 0), ("citm_catalog.json", 0), ("amazon_cellphones.ndjson", 2), ("twitter.json", 2)]:
-        data = np.fromfile(os.path.join(O.JSONEXAMPLES, name), dtype=np.uint8)
+        data = np.frombuffer(O.jsonexample(name), dtype=np.uint8)
         a, h = ice.stage1(data, mode), has.stage1(data, mode)
         assert O.same_stage1(a, h)
         me, mo = ice.minify(data)

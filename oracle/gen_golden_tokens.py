@@ -79,7 +79,7 @@ def main():
                      "string_buf": bytes(sb).hex()})
     files = []
     for name in ("twitter.json", "citm_catalog.json"):
-        d = open(os.path.join(O.JSONEXAMPLES, name), "rb").read()
+        d = O.jsonexample(name)
         err, types, pay, sb = ref.dom_tape(d)
         assert err == 0
         isd = np.array([chr(t) == "d" for t in types])

@@ -1,10 +1,13 @@
 """ctypes bindings for the two CPU checkers under oracle/ (test infrastructure only).
 
   port : oracle/libsj_oracle.so    -- our byte-at-a-time C restatement (always built)
-  ref  : oracle/_ref/libsj_ref.so  -- the unmodified reference compiled from
-                                      /root/reference/singleheader (may be absent)
+  ref  : oracle/_ref/libsj_ref.so  -- the unmodified reference compiled from its
+                                      singleheader sources (may be absent)
+
+and the reference's own sample documents (jsonexample), stored xz-compressed under tests/golden/jsonexamples/.
 """
 import ctypes as C
+import lzma
 import os
 import subprocess
 
@@ -14,7 +17,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 PORT_SO = os.path.join(ORACLE_DIR, "libsj_oracle.so")
 REF_SO = os.path.join(ORACLE_DIR, "_ref", "libsj_ref.so")
-JSONEXAMPLES = os.path.join(ORACLE_DIR, "_ref", "jsonexamples")
+JSONEXAMPLES = os.path.join(ROOT, "tests", "golden", "jsonexamples")
+
+
+def jsonexample(name):
+    """bytes of one of the reference's sample documents: twitter.json, citm_catalog.json, amazon_cellphones.ndjson"""
+    with lzma.open(os.path.join(JSONEXAMPLES, name + ".xz")) as f:
+        return f.read()
 
 SUCCESS, CAPACITY, MEMALLOC, UTF8_ERROR, EMPTY, UNESCAPED_CHARS, UNCLOSED_STRING, UNEXPECTED_ERROR = 0, 1, 2, 11, 13, 14, 15, 24
 REGULAR, STREAMING_PARTIAL, STREAMING_FINAL, JSON_SEQUENCE_PARTIAL, JSON_SEQUENCE_FINAL, COMMA_DELIMITED_PARTIAL, COMMA_DELIMITED_FINAL = range(7)

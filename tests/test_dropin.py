@@ -82,11 +82,7 @@ def h():
 
 def _corpora():
     docs = [b'{"a":[1,2,{"b":"c\\"d"}],"e":null,"u":"\xc3\xa9"}', bytes(corpus.random_json(200000, seed=3)), bytes(corpus.random_json(1 << 20, seed=4))]
-    for name in ("twitter.json", "citm_catalog.json"):
-        path = os.path.join(O.JSONEXAMPLES, name)
-        if os.path.exists(path):
-            docs.append(open(path, "rb").read())
-    return docs
+    return docs + [O.jsonexample(name) for name in ("twitter.json", "citm_catalog.json")]
 
 
 @needs_plugin
@@ -128,19 +124,16 @@ def test_dom_parse_dropin(h):
 @needs_plugin
 @pytest.mark.gpu
 def test_parse_many_dropin(h):
-    path = os.path.join(O.JSONEXAMPLES, "amazon_cellphones.ndjson")
-    streams = [bytes(corpus.ndjson_rows(600000, seed=9)), b'{"a":1} [1,2,3] "x" 12 {"b":[true,false]}  ']
-    if os.path.exists(path):
-        streams.append(open(path, "rb").read())
+    amazon = O.jsonexample("amazon_cellphones.ndjson")
+    streams = [bytes(corpus.ndjson_rows(600000, seed=9)), b'{"a":1} [1,2,3] "x" 12 {"b":[true,false]}  ', amazon]
     for s in streams:
         for batch in (4096, 100000, 1000000):
             c = h.parse_many(0, s, batch)
             g = h.parse_many(1, s, batch)
             assert g[:3] == c[:3], (len(s), batch, g[0], c[0], g[1], c[1])
             assert g[3] >= 1
-    if os.path.exists(path):
-        nd, fe, _, _ = h.parse_many(1, open(path, "rb").read())
-        assert (nd, fe) == (793, 0)  # tests/dom/basictests.cpp L36, L692-708
+    nd, fe, _, _ = h.parse_many(1, amazon)
+    assert (nd, fe) == (793, 0)  # tests/dom/basictests.cpp L36, L692-708
 
 
 @needs_plugin

@@ -77,12 +77,11 @@ def test_golden_minify_and_utf8(parser):
         assert impl.validate_utf8(bytes.fromhex(c["hex"])) == c["valid"], c
 
 
-@pytest.mark.skipif(not os.path.isdir(O.JSONEXAMPLES), reason="reference corpora not staged")
 def test_golden_corpora(parser):
     import torch
     impl = sj.get_active_implementation()
     for f in _load("corpora.json")["files"]:
-        data = np.fromfile(os.path.join(O.JSONEXAMPLES, f["file"]), dtype=np.uint8)
+        data = np.frombuffer(O.jsonexample(f["file"]), dtype=np.uint8).copy()
         r = run_stage1(parser, data, f["mode"])
         assert (r.err, r.n) == (f["err"], f["n"]), f["file"]
         assert hashlib.sha256(r.words().tobytes()).hexdigest() == f["idx_sha256"], f["file"]
@@ -724,7 +723,7 @@ def test_tokens_device_matches_oracle(port):
     assert rc == sj.SUCCESS
     try:
         docs = [bytes(corpus.random_json(rng.randrange(300, 300000), seed=5000 + i)) for i in range(8)]
-        docs += [open(os.path.join(O.JSONEXAMPLES, f), "rb").read() for f in ("twitter.json", "citm_catalog.json")]
+        docs += [O.jsonexample(f) for f in ("twitter.json", "citm_catalog.json")]
         docs += [bytes(corpus.random_json(16 << 20, seed=31337)), b"[]", b"7", b'""', b'{"a":"b"}']
         for _ in range(40):  # documents of adversarial tokens: every scalar and string body the fuzzers produce, errors included
             parts = []
@@ -813,7 +812,7 @@ def test_tokens_device_matches_golden():
             else:
                 assert int(d_type[k]) == 0 and int(d_payload[k]) == c["err"] == res.error and res.first_error_index == k, doc
         for f in g["files"]:
-            doc = open(os.path.join(O.JSONEXAMPLES, f["file"]), "rb").read()
+            doc = O.jsonexample(f["file"])
             rc, d = _tokens_on_device(p, doc)
             res, d_type, d_payload, d_strbuf = p.tokens_device(d)
             types, pay = d_type.cpu().numpy(), d_payload.cpu().numpy().view(np.uint64)

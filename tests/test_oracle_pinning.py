@@ -1,21 +1,21 @@
 """Pins the CPU restatement (oracle/sj_oracle.c) before anything trusts it.
 
  * against the committed golden vectors produced by the unmodified reference
-   (tests/golden/*.json, generator oracle/gen_golden.py) -- runs everywhere;
- * against the live reference (oracle/_ref/libsj_ref.so: icelake AND haswell)
-   on seeded adversarial inputs, all seven stage1 modes -- runs wherever the
-   prebuilt reference .so is present (it ships to the GPU box too).
+   (tests/golden/*.json, generator oracle/gen_golden.py);
+ * against what the reference (icelake AND haswell kernels) returned for
+   seeded adversarial inputs in all seven stage1 modes, recorded in
+   tests/golden/pinning.json.xz (generator oracle/gen_golden_pinning.py,
+   inputs and records in tests/pinning_cases.py).
 """
 import hashlib
 import json
 import os
-import random
 
 import numpy as np
 import pytest
 
 import oracle_lib as O
-from simdjson_b200 import corpus
+import pinning_cases as PC
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -58,10 +58,14 @@ def test_port_matches_golden_utf8(port):
         assert port.validate_utf8(bytes.fromhex(c["hex"])) == c["valid"], c
 
 
-@pytest.mark.skipif(not os.path.isdir(O.JSONEXAMPLES), reason="reference corpora not staged (make -C oracle)")
+@pytest.fixture(scope="module")
+def pinned():
+    return PC.load()
+
+
 def test_port_matches_golden_corpora(port):
     for f in _load("corpora.json")["files"]:
-        data = np.fromfile(os.path.join(O.JSONEXAMPLES, f["file"]), dtype=np.uint8)
+        data = np.frombuffer(O.jsonexample(f["file"]), dtype=np.uint8)
         assert len(data) == f["len"]
         r = port.stage1(data, f["mode"])
         assert (r.err, r.n) == (f["err"], f["n"])
@@ -74,10 +78,7 @@ def test_port_matches_golden_corpora(port):
 def test_amazon_is_793_documents(port):
     """tests/dom/basictests.cpp L36, L692-708: parse_many over amazon_cellphones.ndjson yields 793 docs;
     at stage-1 level: 793 top-level '[' ... ']' rows in streaming_final mode."""
-    path = os.path.join(O.JSONEXAMPLES, "amazon_cellphones.ndjson")
-    if not os.path.exists(path):
-        pytest.skip("reference corpora not staged")
-    data = np.fromfile(path, dtype=np.uint8)
+    data = np.frombuffer(O.jsonexample("amazon_cellphones.ndjson"), dtype=np.uint8)
     r = port.stage1(data, O.STREAMING_FINAL)
     assert r.err == 0 and r.n == 15067
     # count row starts: a '[' structural that is the first structural on its line
@@ -89,78 +90,40 @@ def test_amazon_is_793_documents(port):
     assert starts == 793
 
 
-needs_ref = pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref/libsj_ref.so not built")
+def _same_records(got, want):
+    got = list(got)
+    assert len(got) == len(want), PC.REGENERATE
+    for (ctx, g), w in zip(got, want):
+        assert g == w, (ctx, g, w, PC.REGENERATE)
 
 
-@needs_ref
-@pytest.mark.parametrize("impl", ["icelake", "haswell"])
-def test_port_matches_live_reference_fuzz(port, impl):
-    if impl not in O.ref_impls():
-        pytest.skip(f"{impl} not supported by this host")
-    ref = O.Ref(impl)
-    rng = random.Random(corpus.SEED + (1 if impl == "haswell" else 0))
-    n_cases = 4000
-    for i in range(n_cases):
-        kind = i % 4
-        if kind == 0:
-            b, mode = corpus.adversarial(rng), rng.choice(O.ALL_MODES)
-        elif kind == 1:
-            b, mode = corpus.multi_document(rng), rng.choice([1, 2])
-        elif kind == 2:
-            b, mode = b"\x1e" + corpus.multi_document(rng, sep=b"\x1e"), rng.choice([3, 4])
-        else:
-            b, mode = corpus.multi_document(rng, sep=b","), rng.choice([5, 6])
-        a, r = port.stage1(b, mode), ref.stage1(b, mode)
-        assert O.same_stage1(a, r), (b, mode, a.err, r.err, a.n, r.n)
-        if kind == 0:
-            assert port.minify(b) == ref.minify(b), b
-            assert port.validate_utf8(b) == ref.validate_utf8(b), b
+@pytest.mark.parametrize("impl", PC.FUZZ_IMPLS)
+def test_port_matches_live_reference_fuzz(port, pinned, impl):
+    """stage 1 in all seven modes, minify and validate_utf8 on the seeded inputs drawn for the reference's icelake / haswell
+    kernel, against that kernel's recorded answers"""
+    _same_records(PC.fuzz_records(port, impl), pinned["fuzz"][impl])
 
 
-@needs_ref
-def test_port_matches_live_reference_capacity_and_sizes(port):
-    ref = O.Ref("")
-    doc = b'{"a":[1,2,3],"b":"xyz"}'
+def test_port_matches_live_reference_capacity_and_sizes(port, pinned):
+    """stage 1 / minify / validate_utf8 at every length 0..199 and the block boundaries, against the reference's recorded answers"""
     # len > capacity -> CAPACITY before anything is written (json_structural_indexer.h L195)
-    a, r = port.stage1(doc, 0, capacity=8), ref.stage1(doc, 0, capacity=8)
-    assert a.err == r.err == O.CAPACITY and not a.wrote and not r.wrote
+    assert pinned["sizes"][0] == [O.CAPACITY, O.N_SENTINEL, None]
     # block-boundary lengths
-    rng = random.Random(5)
-    for n in list(range(0, 200)) + [255, 256, 257, 4095, 4096, 4097]:
-        b = bytes(corpus.random_json(max(n, 64)))[:n]
-        for mode in (0, 1, 2):
-            assert O.same_stage1(port.stage1(b, mode), ref.stage1(b, mode)), (n, mode)
-        assert port.minify(b) == ref.minify(b)
-        u = bytes(corpus.random_utf8(max(n, 1), seed=n))[:n]
-        assert port.validate_utf8(u) == ref.validate_utf8(u), n
-        _ = rng
+    _same_records(PC.size_records(port), pinned["sizes"])
 
 
-@needs_ref
-def test_port_matches_live_reference_large(port):
-    ref = O.Ref("")
-    d = corpus.random_json(4 << 20)
-    assert O.same_stage1(port.stage1(d), ref.stage1(d))
-    assert port.minify(d) == ref.minify(d)
-    nd = corpus.ndjson_rows(2 << 20)
-    for mode in (1, 2):
-        assert O.same_stage1(port.stage1(nd, mode), ref.stage1(nd, mode))
+def test_port_matches_live_reference_large(port, pinned):
+    """MiB-sized JSON, NDJSON and UTF-8 text, against the reference's recorded answers"""
+    want = pinned["large"]
     # cut an NDJSON buffer mid-row: streaming_partial must point at the last complete row
-    cut = nd[: (1 << 20) + 123]
-    a, r = port.stage1(cut, 1), ref.stage1(cut, 1)
-    assert O.same_stage1(a, r) and a.err == 0 and a.idx[a.n] < len(cut)
-    u = corpus.random_utf8(1 << 20)
-    assert port.validate_utf8(u) and ref.validate_utf8(u)
-    for pos in (0, len(u) // 2, len(u) - 2):
-        v = u.copy()
-        v[pos] = 0xFF
-        assert not port.validate_utf8(v) and not ref.validate_utf8(v)
+    cut = want[3]
+    assert cut[0] == 0 and cut[3] < (1 << 20) + 123
+    # valid UTF-8, then three corrupted copies
+    assert want[4:] == [True, False, False, False]
+    _same_records(PC.large_records(port), want)
 
 
 # ---------------------------------------------------------------- stage-2-lite (SURVEY.md 8(f) row 4)
-import token_fuzz as TF  # noqa: E402
-
-
 def _tape_view(types, pay):
     """the port's per-structural arrays in the reference's tape order: ':' and ',' have no tape entry"""
     keep = [i for i, t in enumerate(types) if chr(t) not in ":,"]
@@ -203,7 +166,7 @@ def test_port_tokens_match_golden(port):
     for c in g["documents"]:
         _check_doc_against(port, bytes.fromhex(c["doc"]), c["err"], c["types"].encode("latin1"), c["payloads"], bytes.fromhex(c["string_buf"]))
     for f in g["files"]:
-        doc = open(os.path.join(O.JSONEXAMPLES, f["file"]), "rb").read()
+        doc = O.jsonexample(f["file"])
         r = port.stage1(doc)
         err, types, pay, sb, sl, ns, fe = port.tokens(doc, r.idx, r.n)
         t, p = _tape_view(types, pay)
@@ -213,39 +176,32 @@ def test_port_tokens_match_golden(port):
         assert sl == f["string_buf_bytes"] and hashlib.sha256(bytes(sb)).hexdigest() == f["string_buf_sha256"]
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref/libsj_ref.so not built")
-def test_port_tokens_match_live_reference(port):
-    import math
-    rng = random.Random(20260923)
-    for impl in O.ref_impls()[:2]:
-        ref = O.Ref(impl)
-        for _ in range(1500):
-            body, _ = TF.string_body(rng, maxlen=rng.choice([80, 200]))
-            assert port.parse_string(b'"' + body + b'"') == ref.parse_string(body + b'"'), body
-        for _ in range(1500):
-            tok = TF.scalar_token(rng)
-            try:
-                if not math.isfinite(float(tok.decode("latin1"))):
-                    continue  # the reference rejects infinite VALUES (write_float); stage-2-lite does not convert floats
-            except ValueError:
-                pass
-            doc, k = TF.wrap_scalar(tok, rng)
+def test_port_tokens_match_live_reference(port, pinned):
+    """parse_string, one-scalar documents and random documents against the recorded answers of dom::parser::parse"""
+    hint = PC.REGENERATE
+    for impl, (bodies, scalars, docs) in PC.token_inputs().items():
+        want = pinned["tokens"][impl]
+        assert (len(bodies), len(scalars), len(docs)) == tuple(len(want[k]) for k in ("strings", "scalars", "documents")), hint
+        for body, w in zip(bodies, want["strings"]):
+            r, out = port.parse_string(b'"' + body + b'"')
+            assert [r, PC.digest(out)] == w, (body, hint)
+        for (doc, k), (rerr, rtypes, rpay) in zip(scalars, want["scalars"]):
             r = port.stage1(doc)
-            rerr, rtypes, rpay, _sb = ref.dom_tape(doc)
             if r.err != 0:
-                assert rerr == r.err, doc
+                assert rerr == r.err, (doc, hint)
                 continue
             err, types, pay, *_ = port.tokens(doc, r.idx, r.n)
             if rerr == 0:
                 t, p = _tape_view(types, pay)
-                assert err == 0 and t == bytes(rtypes), doc
-                for i, ch in enumerate(t):
-                    if chr(ch) in '"lu':
-                        assert int(p[i]) == int(rpay[i]), doc
+                assert err == 0 and t == rtypes.encode("latin1"), (doc, hint)
+                assert PC.tape_record(np.frombuffer(t, dtype=np.uint8), p)[2] == rpay, (doc, hint)
             else:
-                assert types[k] == 0 and int(pay[k]) == rerr and err == rerr, (doc, err, int(pay[k]), rerr)
-        for i in range(12):
-            doc = bytes(corpus.random_json(rng.randrange(500, 60000), seed=777 + i))
-            rerr, rtypes, rpay, rsb = ref.dom_tape(doc)
-            keep = {str(j): int(rpay[j]) for j, t in enumerate(rtypes) if chr(t) in '"lu'}
-            _check_doc_against(port, doc, rerr, bytes(rtypes), keep, bytes(rsb))
+                assert types[k] == 0 and int(pay[k]) == rerr and err == rerr, (doc, err, int(pay[k]), rerr, hint)
+        for doc, (rerr, *rtape, rsb_len, rsb) in zip(docs, want["documents"]):
+            r = port.stage1(doc)
+            assert r.err == 0
+            err, types, pay, sb, sl, ns, fe = port.tokens(doc, r.idx, r.n)
+            assert err == 0 and fe == 0xFFFFFFFF, (doc[:80], err)
+            t, p = _tape_view(types, pay)
+            assert rerr == 0 and PC.tape_record(np.frombuffer(t, dtype=np.uint8), p) == rtape, (doc[:80], hint)
+            assert [sl, PC.digest(sb)] == [rsb_len, rsb], (doc[:80], hint)

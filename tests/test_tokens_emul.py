@@ -48,7 +48,7 @@ def test_token_functions_match_oracle(emu):
     port = O.Port()
     rng = random.Random(99)
     docs = [bytes(corpus.random_json(rng.randrange(300, 200000), seed=4000 + i)) for i in range(10)]
-    docs += [open(os.path.join(O.JSONEXAMPLES, f), "rb").read() for f in ("twitter.json", "citm_catalog.json")] if os.path.isdir(O.JSONEXAMPLES) else []
+    docs += [O.jsonexample(f) for f in ("twitter.json", "citm_catalog.json")]
     # documents made of adversarial tokens: every scalar kind and string body the fuzzers produce, errors included
     for _ in range(60):
         parts = []
